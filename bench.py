@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200 hot path (see BASELINE.json / SURVEY.md 8d).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--batch B]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--batch B] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path -- CKKS Evaluator::multiply + relinearize_inplace -- over one batch of synthetic
 uniform-random ciphertexts (as native/bench does: bench.h:195-270) that is already resident in HBM.  Under torchrun
@@ -246,6 +246,28 @@ def fail(msg):
     os._exit(3)
 
 
+def dump_outputs(path, out, np, max_ciphertexts=8, max_coeffs=4096):
+    """Write a fixed sample of the device-resident result out[batch][2][L][n] (residue words below 2^63) to path/*.npy, so that
+    two builds can be compared output for output: the same seeded ciphertext and coefficient indices on every run, the first and
+    last ciphertext always among them.  float64 holds 53 bits, so each word is stored exactly as its high and low 32 bits
+    (multiply_relinearize_hi32.npy, multiply_relinearize_lo32.npy, shape [ciphertexts][2][L][coefficients]); the sampled indices
+    are written beside them.  At most 8 x 2 x L x 4096 words, 32 MB for L = 31."""
+    import torch
+
+    B, n = out.shape[0], out.shape[-1]
+    rng = np.random.default_rng(0xD0)
+    inner = rng.choice(np.arange(1, B - 1), size=min(max(B - 2, 0), max_ciphertexts - 2), replace=False)
+    cts = sorted({0, B - 1} | {int(i) for i in inner})
+    cols = np.sort(rng.choice(n, size=min(n, max_coeffs), replace=False))
+    sample = out[torch.tensor(cts, device=out.device)][..., torch.from_numpy(cols).to(out.device)]
+    words = sample.cpu().numpy().view(np.uint64)
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "multiply_relinearize_hi32.npy"), (words >> np.uint64(32)).astype(np.float64))
+    np.save(os.path.join(path, "multiply_relinearize_lo32.npy"), (words & np.uint64(0xFFFFFFFF)).astype(np.float64))
+    np.save(os.path.join(path, "sample_ciphertexts.npy"), np.array(cts, dtype=np.float64))
+    np.save(os.path.join(path, "sample_coefficients.npy"), cols.astype(np.float64))
+
+
 def timed(torch, fn, steps, warmup=1):
     for _ in range(warmup):
         fn()
@@ -487,7 +509,11 @@ def main():
                     help="key switching: 0 = 64-bit digit transforms, 1 = automatic (library default: the integer convolution on auxiliary "
                          "primes from 6 digits on), 2 = the integer path at every level")
     ap.add_argument("--scratch-gib", type=float, default=0.0, help="key-switching scratch budget (0: what the device has left, at most 64 GiB)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of the last timed step's output ciphertexts to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     wl = dict(WORKLOADS[args.workload])
     if args.batch:
         wl["batch"] = args.batch
@@ -601,6 +627,8 @@ def main():
             if not (to_np(out[i]) == want).all():
                 fail(f"{args.workload} ciphertext {i} of the timed run differs from the reference")
         verified = {"indices": idx, "ok": True, "chunk": chunk, "chunks_per_step": -(-B // chunk), "against": against}
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, np)
 
     # end-of-run gather (the only collective besides the key broadcast): one 64-bit digest per ciphertext of this rank's last step
     from seal_b200.shard import digest as ct_digest, gather_digests

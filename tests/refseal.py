@@ -2,13 +2,18 @@
 C wrapper oracle/ref_capi.{h,cpp}.  TEST INFRASTRUCTURE ONLY: imported by tests/, __graft_entry__.smoke() and
 bench.py's cpu_baseline / --impl reference legs; the product never loads it.
 """
+import atexit
+import base64
 import ctypes as C
+import hashlib
+import json
 import os
 
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB_PATH = os.path.join(_HERE, "..", "oracle", "_ref", "libsealref.so")
+_RECORDED_PATH = os.path.join(_HERE, "golden", "reference_results.json")
 
 BFV, CKKS, BGV = 1, 2, 3
 _u64p = C.POINTER(C.c_uint64)
@@ -90,6 +95,148 @@ def lib():
 def _p(a):
     assert a.dtype == np.uint64 and a.flags["C_CONTIGUOUS"]
     return a.ctypes.data_as(_u64p)
+
+
+# ------------------------------------------------------------------------------------------- recorded results ----
+# Tests that only compare with the reference's results run everywhere: through Replay, a call is answered by the live library
+# when oracle/_ref is built, and otherwise from tests/golden/reference_results.json, which holds, per call (keyed by the context,
+# the method and a digest of every argument), the SHA-256 digest of the result, and the result itself for the methods whose
+# results the tests feed to other code (_DATA_METHODS).  A digest-only result (Recorded) compares equal to exactly the words the
+# reference returned.  With SEAL_B200_RECORD_REFERENCE=1 and the live library, the calls a test run makes are added to the file;
+# a live result that contradicts the file fails.
+_DATA_METHODS = {"secret_key", "bfv_encrypt", "batch_codec", "ct_save", "seeded_ct_stream"}
+_recorded = None
+_record = os.environ.get("SEAL_B200_RECORD_REFERENCE") == "1"
+
+
+def _bytes_digest(b):
+    return hashlib.sha256(b).hexdigest()[:40]
+
+
+class Recorded:
+    """A reference result known by the digest of its bytes only; `x == recorded` is true iff x has exactly those bytes"""
+
+    __array_ufunc__ = None  # ndarray == Recorded defers to Recorded.__eq__
+    __hash__ = None
+
+    def __init__(self, digest):
+        self.digest = digest
+
+    def view(self, *_):  # the digest covers the raw bytes, whatever dtype they are viewed as
+        return self
+
+    def __eq__(self, other):
+        return _Match(_digest_of(other) == self.digest)
+
+    def __ne__(self, other):
+        return _Match(_digest_of(other) != self.digest)
+
+
+class _Match:
+    def __init__(self, ok):
+        self.ok = ok
+
+    def all(self):
+        return self.ok
+
+
+def _digest_of(x):
+    if isinstance(x, Recorded):
+        return x.digest
+    if isinstance(x, bytes):
+        return _bytes_digest(x)
+    return _bytes_digest(np.ascontiguousarray(x).tobytes())
+
+
+def _encode(r, full):
+    if r is None:
+        return {"none": 1}
+    if isinstance(r, (tuple, list)):
+        return {"seq": [_encode(x, full) for x in r], "tuple": isinstance(r, tuple)}
+    if isinstance(r, (bytes, np.ndarray)):
+        raw = r if isinstance(r, bytes) else np.ascontiguousarray(r).tobytes()
+        e = {"digest": _bytes_digest(raw)}
+        if full:
+            e["b64"] = base64.b64encode(raw).decode()
+            if isinstance(r, np.ndarray):
+                e["dtype"], e["shape"] = r.dtype.str, list(r.shape)
+        return e
+    return {"v": r.item() if isinstance(r, np.generic) else r}
+
+
+def _decode(e):
+    if "none" in e:
+        return None
+    if "seq" in e:
+        s = [_decode(x) for x in e["seq"]]
+        return tuple(s) if e["tuple"] else s
+    if "digest" in e:
+        if "b64" not in e:
+            return Recorded(e["digest"])
+        raw = base64.b64decode(e["b64"])
+        return np.frombuffer(raw, dtype=e["dtype"]).reshape(e["shape"]).copy() if "dtype" in e else raw
+    return e["v"]
+
+
+def _store():
+    global _recorded
+    if _recorded is None:
+        try:
+            with open(_RECORDED_PATH) as f:
+                _recorded = json.load(f)
+        except FileNotFoundError:
+            _recorded = {}
+        if _record:
+            atexit.register(_save)
+    return _recorded
+
+
+def _save():
+    with open(_RECORDED_PATH, "w") as f:
+        f.write("{\n" + ",\n".join(f"{json.dumps(k)}: {json.dumps(v, sort_keys=True)}" for k, v in sorted(_recorded.items())) + "\n}\n")
+
+
+def _call_key(spec, name, args, kw):
+    parts = [repr(spec), name]
+    for a in list(args) + [kw[k] for k in sorted(kw)]:
+        parts.append(_digest_of(a) if isinstance(a, (np.ndarray, bytes, Recorded)) else repr(a))
+    return _bytes_digest("|".join(parts).encode())
+
+
+def _replayed(spec, name, args, kw, live):
+    """the live result (checked against, or with recording added to, the recorded one) or the recorded result"""
+    store, key = _store(), _call_key(spec, name, args, kw)
+    if live is None:
+        if key not in store:
+            raise KeyError(f"no recorded reference result for {name}{spec}; record it with SEAL_B200_RECORD_REFERENCE=1 where "
+                           f"oracle/_ref is built")
+        return _decode(store[key])
+    r = live(*args, **kw)
+    e = _encode(r, name in _DATA_METHODS)
+    if key in store:
+        assert store[key] == e, f"the live reference's {name}{spec} differs from {_RECORDED_PATH}"
+    elif _record:
+        store[key] = e
+    return r
+
+
+class Replay:
+    """RefContext's methods, answered live when the reference library is built and from the recorded results otherwise"""
+
+    def __init__(self, scheme, n, moduli, plain_modulus=0, seed=0x5EA1):
+        self._spec = (scheme, n, [int(q) for q in moduli], int(plain_modulus), seed)
+        self._live = RefContext(scheme, n, moduli, plain_modulus, seed) if available() else None
+
+    def __getattr__(self, name):
+        if name.startswith("_") or not callable(getattr(RefContext, name, None)):
+            raise AttributeError(name)
+        live = getattr(self._live, name) if self._live is not None else None
+        return lambda *args, **kw: _replayed(self._spec, name, args, kw, live)
+
+
+def replay(fn, *args):
+    """one of this module's context-free functions (coeff_modulus_create, plain_modulus_batching, ...), live or recorded"""
+    return _replayed((), fn.__name__, args, {}, fn if available() else None)
 
 
 def coeff_modulus_create(n, bits):

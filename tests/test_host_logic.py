@@ -198,17 +198,16 @@ def test_blake2b_matches_hashlib():
         assert out.tobytes() == hashlib.blake2b(msg, digest_size=32).digest()
 
 
-@pytest.mark.skipif(not __import__("refseal").available(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("scheme", ["bfv", "ckks", "bgv"])
 def test_parms_id_matches_reference(scheme):
     import refseal as R
 
     P = _probe()
     n = 1024
-    mods = R.coeff_modulus_create(n, [40, 41, 42, 43])
+    mods = R.replay(R.coeff_modulus_create, n, [40, 41, 42, 43])
     sid = {"bfv": R.BFV, "ckks": R.CKKS, "bgv": R.BGV}[scheme]
-    t = 0 if scheme == "ckks" else R.plain_modulus_batching(n, 17)
-    rc = R.RefContext(sid, n, mods, t)
+    t = 0 if scheme == "ckks" else R.replay(R.plain_modulus_batching, n, 17)
+    rc = R.Replay(sid, n, mods, t)
     q = np.array(mods, dtype=np.uint64)
     for L in (4, 3, 2, 1):  # 4 = the key level
         out = np.zeros(4, dtype=np.uint64)
@@ -216,15 +215,14 @@ def test_parms_id_matches_reference(scheme):
         assert tuple(int(x) for x in out) == rc.parms_id(L)
 
 
-@pytest.mark.skipif(not __import__("refseal").available(), reason="oracle/_ref not built")
 def test_ciphertext_inspect_vs_reference_stream():
     import refseal as R
     import seal_b200 as S
     from common import rand_ct
 
     n = 256
-    mods = R.coeff_modulus_create(n, [40, 41, 42])
-    rc = R.RefContext(R.CKKS, n, mods)
+    mods = R.replay(R.coeff_modulus_create, n, [40, 41, 42])
+    rc = R.Replay(R.CKKS, n, mods)
     rng = np.random.default_rng(6)
     for L, size in ((2, 2), (1, 3)):
         data = rand_ct(rng, mods, n, size, L)
