@@ -161,7 +161,12 @@ int sb200_kswitch_key_load(sb200_context *ctx, const uint8_t *stream, size_t len
 
 /* ---- device-resident batch operations (stream = cudaStream_t, may be NULL) ----------------------------------
  * Output slabs must not alias input slabs unless noted: multiply_relinearize may write over d_a or d_b, add/sub/negate/multiply_plain
- * may run in place; relinearize / rescale / mod_switch / apply_galois change the layout and reject aliasing. */
+ * may run in place; relinearize / rescale / mod_switch / apply_galois change the layout and reject aliasing.
+ * The *_host variants stage the batch through the device in chunks (SB200_LIMIT_HOST_STAGE_BYTES; a batch of 4 or more always
+ * takes at least two).  When the batch fits one chunk, host output and input buffers may overlap in any way.  With several chunks
+ * the output may overlap an input only exactly in place (h_out == that input) with an output no larger than that input, as in
+ * add / sub / negate, multiply_plain, relinearize, apply_galois or rescale; any other overlap returns SB200_E_INVALID_ARG before
+ * anything is copied. */
 /* Evaluator::transform_to_ntt_inplace / transform_from_ntt_inplace (evaluator.cpp:2289-2382) */
 int sb200_ntt_forward(sb200_context *ctx, size_t L, size_t size, size_t batch, uint64_t *d_data, void *stream);
 int sb200_ntt_inverse(sb200_context *ctx, size_t L, size_t size, size_t batch, uint64_t *d_data, void *stream);
